@@ -2,6 +2,7 @@
 """bench.py — headline benchmark of the librosa FFT time-frequency hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|cfg3|cfg4|cfg5|stats|speech400]
+                    [--dump-outputs DIR]
 
 Metric (BASELINE.json): mel-spectrogram frames/sec, n_fft=2048, hop=512, n_mels=128, float32, on
 BASELINE.json configs[1] — batch = 1024 clips x 10 s mono @ 22050 Hz per GPU.  One "step" is one pass of
@@ -19,6 +20,10 @@ One JSON line on stdout (rank 0).  Extra keys beyond the base contract:
   secondary     device-resident ms / frames/s / roofline of BASELINE.json configs 3, 4, 5 (per-GPU shards) and of the
                 n_fft = 400 speech front end (`speech400`, mixed-radix kernel; not a BASELINE.json config)
   clocks        NVML samples taken during the timed region
+
+--dump-outputs DIR writes what the last timed step returned (rank 0's shard) as DIR/<name>.npy, float32: whole
+clips picked by a fixed seed, as many as fit in 64 MB; complex spectra get a trailing (real, imag) axis.  The
+inputs depend only on the arguments, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -54,6 +59,9 @@ WORKLOADS = {
                       desc="1024 clips x10s mono sr=16000 -> melspectrogram n_fft=400 hop=160 n_mels=80 per GPU"),
 }
 METRIC = "mel-spectrogram frames/sec (n_fft=2048,hop=512,n_mels=128)"
+OUTPUT_NAMES = {"mel": "melspectrogram", "stft": "stft", "mfcc": "mfcc", "centroid": "spectral_centroid",
+                "roundtrip": "istft"}
+DUMP_BYTES = 60 * 10**6         # under 64 MB however MB is counted, .npy header included
 
 
 def n_frames(n, n_fft, hop):
@@ -348,18 +356,19 @@ def make_steps(lb, w, dev, host):
     kw, op, sr = w["kw"], w["op"], w["sr"]
 
     def step_resident():
+        """One step on the device-resident batch; returns the result (a DeviceArray the caller frees)."""
         if op == "mel":
-            lb.feature.melspectrogram(y=dev, sr=sr, **kw).free()
-        elif op == "stft":
-            lb.stft(dev, **kw).free()
-        elif op == "mfcc":
-            lb.feature.mfcc(y=dev, sr=sr, **kw).free()
-        elif op == "centroid":
-            lb.feature.spectral_centroid(y=dev, sr=sr, **kw).free()
-        else:
-            D = lb.stft(dev, **kw)
-            lb.istft(D, hop_length=kw["hop_length"], length=w["n"]).free()
-            D.free()
+            return lb.feature.melspectrogram(y=dev, sr=sr, **kw)
+        if op == "stft":
+            return lb.stft(dev, **kw)
+        if op == "mfcc":
+            return lb.feature.mfcc(y=dev, sr=sr, **kw)
+        if op == "centroid":
+            return lb.feature.spectral_centroid(y=dev, sr=sr, **kw)
+        D = lb.stft(dev, **kw)
+        y = lb.istft(D, hop_length=kw["hop_length"], length=w["n"])
+        D.free()
+        return y
 
     def step_e2e(src=None):
         y = host if src is None else src
@@ -374,6 +383,23 @@ def make_steps(lb, w, dev, host):
         return lb.istft(lb.stft(y, **kw), hop_length=kw["hop_length"], length=w["n"])
 
     return step_resident, step_e2e
+
+
+def dump_outputs(out, name, directory):
+    """Copy a seeded sample of whole clips of the device result ``out`` (clips leading) to DIR/<name>.npy."""
+    from librosa_b200 import _native as nat
+
+    n_clips = out.shape[0]
+    clip_bytes = out.nbytes // n_clips
+    clips = np.sort(np.random.default_rng(0).choice(n_clips, min(n_clips, DUMP_BYTES // clip_bytes), replace=False))
+    rows = []
+    for c in clips:
+        view = nat.DeviceArray(out.ctx, out.ptr + int(c) * clip_bytes, out.shape[1:], out.dtype, layout=out.layout,
+                               owner=False)
+        host = view.get(out=np.empty(view._mem_shape(), out.dtype))
+        rows.append(np.stack([host.real, host.imag], axis=-1) if host.dtype.kind == "c" else host)
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, f"{name}.npy"), np.stack(rows).astype(np.float32))
 
 
 KERNEL_NAMES = {"mel": "fwd_kernel<10,32,16,MODE_MEL>", "stft": "fwd_kernel<.,.,.,MODE_STFT>",
@@ -417,21 +443,25 @@ def run_ours(args, w, rank, world, local_rank):
     peak, peak_src = measured_peak()
 
     def resident(wl, steps, warmup, sample_clocks):
-        """Device-resident timing of one workload: (ms per step max over ranks, launches, clocks, frames per GPU)."""
+        """Device-resident timing of one workload: (ms per step max over ranks, launches, clocks, frames per GPU,
+        result of the last timed step)."""
         T = n_frames(wl["n"], wl["kw"]["n_fft"], wl["kw"]["hop_length"])
         host = lb.pinned_empty((wl["clips"], wl["n"]), np.float32)
         host[...] = make_batch(wl, rank)
         dev = ctx.to_device(host)
         step_resident, step_e2e = make_steps(lb, wl, dev, host)
         for _ in range(max(3, warmup)):
-            step_resident()
+            step_resident().free()
         barrier()
         sampler = ClockSampler(local_rank) if (rank == 0 and sample_clocks) else None
         launches0 = ctx.launch_count
         e0, e1 = ctx.event(), ctx.event()
+        out = None
         e0.record()
         for _ in range(steps):
-            step_resident()
+            if out is not None:
+                out.free()
+            out = step_resident()
         e1.record()
         ms = e0.elapsed_ms(e1)
         barrier()
@@ -439,7 +469,7 @@ def run_ours(args, w, rank, world, local_rank):
         clocks = sampler.stop() if sampler else None
         ms_per_step = max_over_ranks(ms) / steps
         return dict(ms_per_step=ms_per_step, launches=launches, clocks=clocks, frames=wl["clips"] * T, host=host,
-                    dev=dev, step_e2e=step_e2e)
+                    dev=dev, step_e2e=step_e2e, out=out)
 
     def roofline_of(wl, ms_per_step, name):
         alg_bytes = algorithmic_bytes_per_step(wl)
@@ -454,6 +484,9 @@ def run_ours(args, w, rank, world, local_rank):
     ms_per_step, launches, clocks, frames_per_step = r["ms_per_step"], r["launches"], r["clocks"], r["frames"]
     host, dev, step_e2e = r["host"], r["dev"], r["step_e2e"]
     value = world * frames_per_step / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(r["out"], OUTPUT_NAMES[w["op"]], args.dump_outputs)
+    r["out"].free()
 
     # ---- end to end through the public call with host buffers (H2D + D2H inside the timed region)
     def time_e2e(src, steps):
@@ -553,6 +586,7 @@ def run_ours(args, w, rank, world, local_rank):
                 secondary.append({"name": name, "error": repr(exc)[:200]})
                 continue
             rr["dev"].free()
+            rr["out"].free()
             ms2 = rr["ms_per_step"]
             secondary.append({"name": name, "workload": wl["desc"], "metric": f"{wl['op']} frames/sec",
                               "value": world * rr["frames"] / (ms2 * 1e-3), "unit": "frames/s", "ms_per_step": ms2,
@@ -629,7 +663,11 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-secondary", action="store_true", help="skip the cfg3 / cfg4 / cfg5 / speech400 secondary numbers")
     ap.add_argument("--no-join", action="store_true", help="skip the NCCL scatter -> mel -> gather leg (N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's result to "
+                                                           "DIR/<name>.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

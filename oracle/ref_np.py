@@ -6,10 +6,10 @@ TEST INFRASTRUCTURE ONLY.  Nothing under ``librosa_b200/`` imports this module; 
 legs as the checker and as the timed CPU port.  The product path is the CUDA library and fails
 loudly if it is missing.
 
-Parity status: PINNED.  Every function below is checked (a) against the unmodified reference
-imported from /root/reference in the build container (``tests/test_oracle_vs_reference.py``, via
-``tools/ref_shim.py``) and (b) against committed fixtures generated from that reference
-(``tests/golden/*.npz`` written by ``tools/make_golden.py``), which travel to the GPU box.
+Parity status: PINNED.  Every function below is checked against committed fixtures generated from the
+unmodified reference (``tests/golden/*.npz`` written by ``tools/make_golden.py`` through
+``tools/ref_shim.py``): bit for bit in ``tests/test_oracle_vs_reference.py``, within a tolerance that
+absorbs SIMD / BLAS differences between hosts in ``tests/test_oracle_golden.py``.
 
 The reference is pure Python; its arithmetic lives in third-party libraries that are not under
 /root/reference and are called here exactly as the reference calls them:

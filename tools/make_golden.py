@@ -1,11 +1,13 @@
-"""Generate tests/golden/hotpath_v1.npz (tests/cases.py) and tests/golden/features_v1.npz
-(tests/feature_cases.py) by running the cases through the UNMODIFIED reference.
+"""Generate tests/golden/hotpath_v1.npz (tests/cases.py), tests/golden/features_v1.npz
+(tests/feature_cases.py) and tests/golden/reference_exact_v1.npz (tests/reference_outputs.py) by running
+the cases through the UNMODIFIED reference.
 
 Build-container only (needs /root/reference; see tools/ref_shim.py).  The fixtures travel to the GPU box,
 where /root/reference does not exist.  Also stores a handful of constant tables (mel bases, window
 sum-square, mel-scale known answers) produced by the reference.
 
-    python tools/make_golden.py
+    python tools/make_golden.py            # all three fixtures
+    python tools/make_golden.py exact      # only reference_exact_v1.npz
 """
 from __future__ import annotations
 
@@ -88,7 +90,23 @@ def main():
     path = os.path.join(ROOT, "tests", "golden", "features_v1.npz")
     np.savez_compressed(path, **feats)
     print("wrote", path, os.path.getsize(path), "bytes")
+    write_reference_exact(ref)
+
+
+def write_reference_exact(ref):
+    """Records (shape, SHA-256, seeded sample) of the outputs tests/test_oracle_vs_reference.py pins bit for bit."""
+    import reference_outputs
+
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        outputs = reference_outputs.all_groups(ref)
+    path = os.path.join(ROOT, "tests", "golden", "reference_exact_v1.npz")
+    np.savez_compressed(path, **reference_outputs.record(outputs))
+    print("wrote", path, os.path.getsize(path), "bytes;", len(outputs), "outputs")
 
 
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["exact"]:
+        write_reference_exact(ref_shim.load_reference())
+    else:
+        main()

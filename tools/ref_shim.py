@@ -1,9 +1,8 @@
 """Import the *unmodified* reference librosa from /root/reference in this container.
 
 Build-container-only helper (the GPU box has no /root/reference). It is used by
-``tools/make_golden.py`` to generate the committed fixtures under ``tests/golden/`` and by
-``tests/test_oracle_vs_reference.py`` (skipped when the reference tree is absent) to pin the
-``oracle/`` restatement against the real thing.
+``tools/make_golden.py`` to generate the committed fixtures under ``tests/golden/``, against which
+the tests pin the ``oracle/`` restatement; no test imports the reference itself.
 
 librosa imports four modules at import time that are missing from the image and never called on
 the stft / istft / melspectrogram / mfcc path (``lazy_loader``, ``soundfile``, ``soxr``, ``pooch``);
