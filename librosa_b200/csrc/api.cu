@@ -744,7 +744,7 @@ extern "C" int b2l_plan_create(b2l_ctx* c, const b2l_plan_desc* d, b2l_plan** ou
     }
   }
   if (d->n_mfcc > 0) {
-    // transposed and zero padded to 8-coefficient groups: dctT[m][8*KG] (dct_clamp_kernel)
+    // transposed and zero padded to 8-coefficient groups: dctT[m][8*KG] (dct_clamp4_kernel)
     const int KP = (d->n_mfcc + 7) / 8 * 8;
     std::vector<float> dct((size_t)d->n_mels * KP, 0.0f);
     for (int k = 0; k < d->n_mfcc; ++k)
@@ -807,8 +807,8 @@ static int ensure_clip_max(b2l_ctx* c, size_t n_clips) {
 }
 
 // MelRow table for warps that process H mel rows at a time (see MelRow / MelLayout in common.cuh), plus the
-// work-item lists of the `hw` warps of a half: items sorted by length and dealt longest-first to the least
-// loaded warp (the bands of the highest mel rows are ten times longer than those of the lowest).
+// work-item lists of the `hw` warps of a half: items dealt round-robin in row order, which keeps neighbouring
+// rows (whose bands overlap in shared memory) on warps that run at the same time.
 static int get_row_table(b2l_ctx* c, const b2l_plan* p, int H, int hw, const b2l_plan::RowTable** out) {
   const int key = H * 64 + hw;
   auto it = p->row_tables.find(key);
@@ -821,7 +821,6 @@ static int get_row_table(b2l_ctx* c, const b2l_plan* p, int H, int hw, const b2l
   const int n_items = n_rows / H;
   std::vector<MelRow> rows(n_rows);
   std::vector<float> w;
-  std::vector<int> item_quads(n_items, 0);
   for (int item = 0; item < n_items; ++item) {
     std::vector<int> start(H), lenp(H);
     int quads = 0;
@@ -840,7 +839,6 @@ static int get_row_table(b2l_ctx* c, const b2l_plan* p, int H, int hw, const b2l
       }
       quads = std::max(quads, (lenp[j] + 3) / 4);
     }
-    item_quads[item] = quads;
     for (int j = 0; j < H; ++j) {
       const int m = item * H + j;
       MelRow r;
@@ -856,27 +854,8 @@ static int get_row_table(b2l_ctx* c, const b2l_plan* p, int H, int hw, const b2l
       rows[m] = r;
     }
   }
-  // longest-processing-time-first: cost of an item = its trip count + a fixed part (row fetch, stores)
-  std::vector<int> idx(n_items);
-  for (int i = 0; i < n_items; ++i) idx[i] = i;
-  // B2L_MEL_LPT=1: longest-first deal to the least loaded warp.  Measured neutral to slightly negative on cfg 2
-  // (1.148 vs 1.139 ms): the natural order, dealt round-robin, keeps neighbouring rows (whose bands overlap
-  // in shared memory) on warps that run at the same time.  Default: round-robin.
-  const char* lpt_env = getenv("B2L_MEL_LPT");
-  const bool round_robin = !(lpt_env && *lpt_env && atoi(lpt_env) != 0);
-  if (!round_robin)
-    std::stable_sort(idx.begin(), idx.end(), [&](int x, int y) { return item_quads[x] > item_quads[y]; });
   std::vector<std::vector<int>> lists(hw);
-  std::vector<int> load(hw, 0);
-  int rr = 0;
-  for (int i : idx) {
-    int best = 0;
-    for (int wv = 1; wv < hw; ++wv)
-      if (load[wv] < load[best]) best = wv;
-    if (round_robin) best = (rr++) % hw;
-    lists[best].push_back(i);
-    load[best] += item_quads[i] + 3;
-  }
+  for (int i = 0; i < n_items; ++i) lists[i % hw].push_back(i);
   size_t list_len = 0;
   for (auto& l : lists) list_len = std::max(list_len, l.size());
   std::vector<unsigned short> order(list_len * hw, (unsigned short)0xffff);
@@ -896,12 +875,6 @@ static int get_row_table(b2l_ctx* c, const b2l_plan* p, int H, int hw, const b2l
 
 // Kernel variants tried in order (first that fits shared memory wins): 116 = 16 warps as two independent
 // 8-warp halves, 16 / 8 = plain CTAs.  B2L_FWD_VARIANT forces one (A/B measurements).
-#ifndef B2L_MEL2_DEFAULT
-#define B2L_MEL2_DEFAULT false
-#endif
-#ifndef B2L_DCT_FPL_DEFAULT
-#define B2L_DCT_FPL_DEFAULT 4
-#endif
 #ifndef B2L_TMEM_DEFAULT
 #define B2L_TMEM_DEFAULT true
 #endif
@@ -950,69 +923,6 @@ static int run_forward(b2l_ctx* c, const b2l_plan* p, int mode, int log_mode, co
   const int n_opt = fwd_variants(cfg, variants);
   FwdArgs a;
   memset(&a, 0, sizeof(a));
-  // melspectrogram, n_fft = 2048, hop = n_fft / 4, no dB epilogue: autonomous frame groups (mel2_kernel.cuh);
-  // B2L_MEL2=0 keeps fwd_kernel
-  {
-    const char* e2 = getenv("B2L_MEL2");
-    const bool forced = getenv("B2L_FWD_VARIANT") && *getenv("B2L_FWD_VARIANT");
-    if (mode == MODE_MEL && !log_mode && p->log2m == 10 && 4 * p->hop == N && !forced &&
-        (e2 && *e2 ? atoi(e2) != 0 : B2L_MEL2_DEFAULT)) {
-      const b2l_plan::RowTable* t = nullptr;
-      int rc = get_row_table(c, p, mel_rows_per_warp(8), 8, &t);
-      if (rc) return rc;
-      const int PRS = ((M + 4 + 31) / 32) * 32 + 8;
-      size_t off = 0;
-      a.off_bar = (int)off; off = align_up(off + 64, 128);
-      a.off_win = (int)off; off = align_up(off + 2 * 8 * sizeof(long long), 128);       // per-row output offsets
-      a.off_melw = (int)off; off = align_up(off + (size_t)t->w_count * 4, 16);
-      a.off_melband = (int)off; off = align_up(off + (size_t)t->n_rows * sizeof(MelRow), 16);
-      a.off_melorder = (int)off; off = align_up(off + (size_t)std::max(1, t->list_len) * 8 * 2, 128);
-      a.off_in = (int)off; off = align_up(off + (size_t)2 * 8 * PRS * 4, 128);           // power tiles of the two halves
-      a.off_xbuf = (int)off; off += (size_t)16 * cfg.xbuf_f2() * 8;
-      if (off <= c->smem_optin) {
-        a.y = d_y;
-        a.clip_stride = y_stride;
-        a.n = (int)n;
-        a.n_clips = (int)n_clips;
-        a.n_fft = N;
-        a.hop = p->hop;
-        a.pad = p->center ? N / 2 : 0;
-        a.pad_mode = p->pad_mode;
-        a.n_frames = (int)T;
-        a.tma_ok = (((uintptr_t)d_y & 7) == 0) && (y_stride % 2 == 0) && (a.pad % 2 == 0);   // 8-byte sample loads
-        a.window = p->d_win_fwd;
-        a.tw = p->d_tw;
-        a.twn = p->d_twn;
-        a.out_r = out_r;
-        a.power_mode = p->power_mode;
-        a.power = p->power;
-        a.n_mels = p->n_mels;
-        a.mel_w_count = t->w_count;
-        a.mel_w = t->d_w;
-        a.mel_rows = t->d_rows;
-        a.n_mel_rows = t->n_rows;
-        a.mel_order = t->d_order;
-        a.mel_list_len = t->list_len;
-        a.status = c->d_status;
-        const long long total_frames = (long long)n_clips * T;
-        long long grid = c->sm_count;
-        if (grid * 16 > total_frames) grid = (total_frames + 15) / 16;
-        const long long fpg = (total_frames + grid * 16 - 1) / (grid * 16);
-        if (fpg <= 0x7fffffffLL) {
-          a.tiles_per_clip = (int)fpg;                     // steps: frames per frame group
-          const unsigned long long kkey = (7ULL << 60);
-          if (c->launch_cache.find(kkey) == c->launch_cache.end()) {
-            CUDA_TRY(op(OP_SET_SMEM, 3016, mode, &a, 0, c->smem_optin, c->stream, nullptr));
-            c->launch_cache[kkey] = 1;
-          }
-          CUDA_TRY(op(OP_LAUNCH, 3016, mode, &a, (int)grid, off, c->stream, nullptr));
-          c->launches++;
-          return B2L_OK;
-        }
-      }
-      memset(&a, 0, sizeof(a));
-    }
-  }
   int variant = 0, ft = 0, halves = 1;
   size_t smem = 0;
   const b2l_plan::RowTable* rt = nullptr;
@@ -1034,7 +944,7 @@ static int run_forward(b2l_ctx* c, const b2l_plan* p, int mode, int log_mode, co
     size_t off = 0;
     a.off_win = (int)off; if (!tmem) off = align_up(off + (size_t)N * 4, 16);       // TMEM variants keep these
     a.off_tw = (int)off; if (!tmem) off = align_up(off + (size_t)cfg.tw_count() * 8, 16);   // tables off shared memory
-    a.off_bar = (int)off; off = align_up(off + 64, 16);   // "tile landed" mbarrier per half, TMEM base address, "staging consumed" mbarriers
+    a.off_bar = (int)off; off = align_up(off + 64, 16);   // "tile landed" mbarrier per half, TMEM base address, one more mbarrier per half (initialised only)
     if (t) {
       a.off_melw = (int)off; off = align_up(off + (size_t)t->w_count * 4, 16);
       a.off_melband = (int)off; off = align_up(off + (size_t)t->n_rows * sizeof(MelRow), 16);
@@ -1445,7 +1355,8 @@ static int launch_dct(b2l_ctx* c, const b2l_plan* p, const float* d_L, int64_t n
                       float* d_out, int tiled = 0) {
   const int KG = (p->n_mfcc + 7) / 8;
   if (KG > 16) return fail(B2L_ERR_UNSUPPORTED, "n_mfcc=%d > 128 is not supported", p->n_mfcc);
-  size_t smem = ((size_t)p->n_mels * 8 * KG + 2 * (size_t)p->n_mels * DCT_TILE) * 4;
+  // dct_clamp4_kernel: the DCT table [n_mels][8*KG] and one tile of DCT4_TILE frames in shared memory
+  const size_t smem = (size_t)p->n_mels * (8 * KG + DCT4_TILE) * 4;
   if (smem > c->smem_optin) {
     // too many input rows for the shared-memory tile (e.g. mfcc(S=...) of a 1025-bin spectrogram): generic kernel
     if (tiled) return fail(B2L_ERR_UNSUPPORTED, "n_mels=%d is too large for the fused mfcc path", p->n_mels);
@@ -1457,36 +1368,12 @@ static int launch_dct(b2l_ctx* c, const b2l_plan* p, const float* d_L, int64_t n
     c->launches++;
     return B2L_OK;
   }
-  // frames per lane: 2 halves the shared-memory traffic per FMA (B2L_DCT_FPL=1 selects the two-warp-set form)
-  const char* env = getenv("B2L_DCT_FPL");
-  const int fpl = env && *env ? atoi(env) : B2L_DCT_FPL_DEFAULT;
-  if (fpl == 4) {
-    // four frames per lane, 128-frame tiles, one tile buffer per block (dct_clamp4_kernel)
-    const size_t smem4 = ((size_t)p->n_mels * 8 * KG + 2 * (size_t)p->n_mels * 64) * 4;
-    // two warp sets over the mel rows (B2L_DCT_KS=1: one) when the partial sums fit in the tile buffer
-    const char* ks_env = getenv("B2L_DCT_KS");
-    const int ks = (ks_env && *ks_env ? atoi(ks_env) : 2) == 2 && KG <= 10 && p->n_mels >= 8 * KG ? 2 : 1;   // 640 threads at most; 32*KG*32 partial sums <= 2*n_mels*64 tile words
-    auto dct_clamp4 = ks == 2 ? dct_clamp4_kernel<2> : dct_clamp4_kernel<1>;
-    const int threads4 = KG * 32 * ks;
-    CUDA_TRY(cudaFuncSetAttribute(dct_clamp4, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem4));
-    const int tiles4 = (int)((T + DCT4_TILE - 1) / DCT4_TILE);
-    const long long total4 = (long long)tiles4 * n_clips;
-    int occ4 = 0;
-    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ4, dct_clamp4, threads4, smem4));
-    if (occ4 < 1) return fail(B2L_ERR_CUDA, "DCT kernel does not fit on an SM");
-    long long grid4 = (long long)c->sm_count * occ4;
-    if (grid4 > total4) grid4 = total4;
-    dct_clamp4<<<(int)grid4, threads4, smem4, c->stream>>>(d_L, p->d_dct, clamp ? c->d_clip_max : nullptr,
-                                                                  clamp ? p->top_db : -1.0f, p->n_mels, p->n_mfcc, (int)T,
-                                                                  tiles4, total4, tiled, d_out);
-    CUDA_TRY(cudaGetLastError());
-    c->launches++;
-    return B2L_OK;
-  }
-  auto kern = fpl == 2 ? dct_clamp_kernel<2> : dct_clamp_kernel<1>;
-  const int threads = fpl == 2 ? KG * 32 : KG * 64;
+  // two warp sets over the mel rows when the partial sums fit in the tile buffer
+  const int ks = KG <= 10 && p->n_mels >= 8 * KG ? 2 : 1;   // 640 threads at most; 32*KG*32 partial sums <= 2*n_mels*64 tile words
+  auto kern = ks == 2 ? dct_clamp4_kernel<2> : dct_clamp4_kernel<1>;
+  const int threads = KG * 32 * ks;
   CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const int tiles = (int)((T + DCT_TILE - 1) / DCT_TILE);
+  const int tiles = (int)((T + DCT4_TILE - 1) / DCT4_TILE);
   const long long total = (long long)tiles * n_clips;
   int occ = 0;
   CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, smem));
@@ -1516,7 +1403,7 @@ extern "C" int b2l_mfcc(b2l_ctx* c, const b2l_plan* p, const float* d_y, int64_t
   if (rc) return rc;
   CUDA_TRY(cudaMemsetAsync(c->d_clip_max, 0, (size_t)n_clips * sizeof(unsigned int), c->stream));
   float* scratch = d_logmel;
-  // the log-mel scratch is tiled: [clip][ceil(T/64)][n_mels][64] (see dct_clamp_kernel)
+  // the log-mel scratch is tiled: [clip][ceil(T/64)][n_mels][64] (see dct_clamp4_kernel)
   if (!scratch) CUDA_TRY(cudaMalloc((void**)&scratch, (size_t)n_clips * p->n_mels * ((T + 63) / 64 * 64) * sizeof(float)));
   // mixed-radix frames (mr_kernel): the dB rows go to the scratch in the plain [clip][mel][frame] layout
   const int tiled = p->czt ? 0 : 1;

@@ -7,21 +7,6 @@
 namespace b2l {
 
 // ------------------------------------------------------------------ clamp + DCT (mfcc pass B)
-// in  L   [n_clips][n_mels][T]   log-mel (dB), not yet clamped — or, `tiled`, the mfcc scratch of fwd_kernel:
-//         [n_clips][ceil(T/64)][n_mels][64], every 64-frame tile one contiguous block (full DRAM bursts
-//         instead of 256-byte pieces 4*T bytes apart)
-// out C   [n_clips][n_mfcc][T]   C[k][t] = sum_m dct[k][m] * max(L[m][t], clipmax - top_db)
-// Reference: np.maximum(log_spec, log_spec.max(...) - top_db) (librosa/core/spectrum.py:1881) followed by
-// scipy.fft.dct(S, axis=-2, type, norm)[..., :n_mfcc, :] (* lifter) (librosa/feature/spectral.py:2005-2015);
-// the DCT (any type / norm, lifter folded in) arrives transposed and zero padded: dctT[m][8*KG].
-//
-// Persistent blocks of 2*KG warps walk (clip, 64-frame tile) pairs.  Warp w owns coefficients 8*(w % KG) ..
-// +7 for frames 32*(w / KG) + lane of the tile (one frame per lane: twice the warps of a two-frames-per-lane
-// layout for the same shared memory, which is what hides the shared-memory latency of the short inner loop);
-// DCT rows are warp-uniform float4 loads.  Tiles are double buffered with cp.async (LDGSTS) so the next
-// tile streams in while this one is multiplied; the top_db clamp is applied as the values are read.
-constexpr int DCT_TILE = 64;
-
 __device__ __forceinline__ void cp_async4(void* dst_smem, const void* src) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"((uint32_t)__cvta_generic_to_shared(dst_smem)), "l"(src)
                : "memory");
@@ -34,105 +19,21 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
-// FPL = frames per lane: 1 -> two warp sets per tile (frames 0-31 / 32-63), 2 -> one warp set whose lanes own
-// frames (lane, lane + 32): the two warp-uniform coefficient fetches of a mel row (eight shared-memory
-// wavefronts) then feed 16 FMAs instead of 8 — the kernel is bound by the shared-memory pipe.
-template <int FPL>
-__global__ void dct_clamp_kernel(const float* __restrict__ L, const float* __restrict__ dctT,
-                                 const unsigned int* __restrict__ clip_max, float top_db, int n_mels,
-                                 int n_mfcc, int T, int tiles_per_clip, long long total_tiles, int tiled,
-                                 float* __restrict__ C) {
-  extern __shared__ __align__(16) float s_dyn[];
-  const int KG = FPL == 1 ? blockDim.x >> 6 : blockDim.x >> 5, KP = 8 * KG;   // FPL 1: two warp sets, frames 0-31 / 32-63
-  float* s_dct = s_dyn;                                     // [n_mels][KP]
-  float* s_tile0 = s_dyn + n_mels * KP;                     // 2 x [n_mels][DCT_TILE]
-  const int tile_words = n_mels * DCT_TILE;
-  const int tid = threadIdx.x, lane = tid & 31;
-  const int warp = (tid >> 5) % KG, fhalf = (tid >> 5) / KG;
-  for (int i = tid; i < n_mels * KP; i += blockDim.x) s_dct[i] = dctT[i];
-  const bool vec_ok = (T % 4 == 0) && ((reinterpret_cast<uintptr_t>(L) & 15) == 0);
-
-  auto stage = [&](long long tile, float* buf) {
-    const int clip = (int)(tile / tiles_per_clip);
-    const int t0 = (int)(tile % tiles_per_clip) * DCT_TILE;
-    if (tiled) {
-      // scratch written by fwd_kernel (out_tiled): the tile is one contiguous, 16-byte aligned block
-      const float* Lt = L + ((long long)clip * tiles_per_clip + t0 / DCT_TILE) * tile_words;
-      for (int i = tid; i < tile_words / 4; i += blockDim.x) cp_async16(buf + 4 * i, Lt + 4 * i);
-      cp_async_commit();
-      return;
-    }
-    const float* Lc = L + (long long)clip * n_mels * T + t0;
-    if (vec_ok && t0 + DCT_TILE <= T) {
-      for (int i = tid; i < n_mels * (DCT_TILE / 4); i += blockDim.x) {
-        const int m = i / (DCT_TILE / 4), q = i % (DCT_TILE / 4);
-        cp_async16(buf + m * DCT_TILE + 4 * q, Lc + (long long)m * T + 4 * q);
-      }
-    } else {
-      for (int i = tid; i < tile_words; i += blockDim.x) {
-        const int m = i / DCT_TILE, x = i % DCT_TILE;
-        if (t0 + x < T) cp_async4(buf + i, Lc + (long long)m * T + x);
-        else buf[i] = 0.0f;
-      }
-    }
-    cp_async_commit();
-  };
-
-  long long tile = blockIdx.x;
-  if (tile < total_tiles) stage(tile, s_tile0);
-  int cur = 0;
-  for (; tile < total_tiles; tile += gridDim.x, cur ^= 1) {
-    const long long nxt = tile + gridDim.x;
-    if (nxt < total_tiles) {
-      stage(nxt, s_tile0 + (cur ^ 1) * tile_words);
-      cp_async_wait<1>();
-    } else {
-      cp_async_wait<0>();
-    }
-    __syncthreads();
-    const float* tile_s = s_tile0 + cur * tile_words;
-    const int clip = (int)(tile / tiles_per_clip);
-    const int t0 = (int)(tile % tiles_per_clip) * DCT_TILE;
-    float floor_v = -INFINITY;
-    if (clip_max != nullptr && top_db >= 0.0f) floor_v = key_to_float(clip_max[clip]) - top_db;
-    float acc[8], acc2[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) acc[j] = acc2[j] = 0.0f;
-    const int fl = lane + 32 * (FPL == 1 ? fhalf : 0);   // (first) frame of this lane inside the tile
-#pragma unroll 8
-    for (int m = 0; m < n_mels; ++m) {
-      const float4 d0 = *reinterpret_cast<const float4*>(s_dct + m * KP + 8 * warp);
-      const float4 d1 = *reinterpret_cast<const float4*>(s_dct + m * KP + 8 * warp + 4);
-      const float dv[8] = {d0.x, d0.y, d0.z, d0.w, d1.x, d1.y, d1.z, d1.w};
-      const float x0 = fmaxf(tile_s[m * DCT_TILE + fl], floor_v);
-#pragma unroll
-      for (int j = 0; j < 8; ++j) acc[j] = fmaf(dv[j], x0, acc[j]);
-      if constexpr (FPL == 2) {
-        const float x1 = fmaxf(tile_s[m * DCT_TILE + fl + 32], floor_v);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) acc2[j] = fmaf(dv[j], x1, acc2[j]);
-      }
-    }
-    float* Cc = C + (long long)clip * n_mfcc * T;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const int k = 8 * warp + j;
-      if (k < n_mfcc && t0 + fl < T) Cc[(long long)k * T + t0 + fl] = acc[j];
-      if constexpr (FPL == 2) {
-        if (k < n_mfcc && t0 + fl + 32 < T) Cc[(long long)k * T + t0 + fl + 32] = acc2[j];
-      }
-    }
-    __syncthreads();   // tile consumed before the buffer is refilled two iterations later
-  }
-}
-
-// Four frames per lane, the shipped form.  The loop above is bound by the shared-memory pipe: a warp-uniform
-// 16-byte load of four DCT coefficients costs four wavefronts, so a mel row costs 8 + FPL wavefronts per warp
-// for 8 * FPL FMAs (0.625 per FMA at FPL = 2).  Here a tile is 128 frames (two 64-frame blocks of the tiled
-// scratch, contiguous in memory), lane l owns frames 4l .. 4l+3 — one 16-byte load per mel row — and the 32
-// accumulators of a lane are 16 register pairs fed by packed FMAs (coefficient broadcast, frame pair): 12
-// wavefronts and 16 FFMA2 per mel row and warp, 0.375 wavefronts per FMA.  One tile buffer per block; two blocks
-// per SM alternate between streaming and multiplying (cp.async), which is what the double buffer did before.
+// in  L   [n_clips][n_mels][T]   log-mel (dB), not yet clamped — or, `tiled`, the mfcc scratch of fwd_kernel:
+//         [n_clips][ceil(T/64)][n_mels][64], every 64-frame tile one contiguous block (full DRAM bursts
+//         instead of 256-byte pieces 4*T bytes apart)
+// out C   [n_clips][n_mfcc][T]   C[k][t] = sum_m dct[k][m] * max(L[m][t], clipmax - top_db)
+// Reference: np.maximum(log_spec, log_spec.max(...) - top_db) (librosa/core/spectrum.py:1881) followed by
+// scipy.fft.dct(S, axis=-2, type, norm)[..., :n_mfcc, :] (* lifter) (librosa/feature/spectral.py:2005-2015);
+// the DCT (any type / norm, lifter folded in) arrives transposed and zero padded: dctT[m][8*KG].
+//
+// Persistent blocks walk (clip, 128-frame tile) pairs; warp w owns coefficients 8*(w % KG) .. +7, DCT rows
+// are warp-uniform float4 loads and the top_db clamp is applied as the values are read.  The loop is bound by
+// the shared-memory pipe: a warp-uniform 16-byte load of four DCT coefficients costs four wavefronts.  A tile is
+// two 64-frame blocks of the tiled scratch, contiguous in memory; lane l owns frames 4l .. 4l+3 — one 16-byte
+// load per mel row — and the 32 accumulators of a lane are 16 register pairs fed by packed FMAs (coefficient
+// broadcast, frame pair): 12 wavefronts and 16 FFMA2 per mel row and warp, 0.375 wavefronts per FMA.  One tile
+// buffer per block; two blocks per SM alternate between streaming and multiplying (cp.async).
 // KS = 2: two warp sets split the mel rows of a tile and add their partial sums through the (then idle) tile
 // buffer — twice the warps per SM (20 for 40 coefficients, five per scheduler) for one more barrier per tile.
 constexpr int DCT4_TILE = 128;

@@ -95,7 +95,7 @@ struct FwdArgs {
   const unsigned short* mel_order;   // [mel_list_len][warps per half]: k-th work item of each warp (0xffff: none)
   int mel_list_len;
   int log_mode;              // 1: write 10*log10(max(amin, S)) - db_sub and track the per-clip max
-  int out_tiled;             // MODE_MEL: out_r is the mfcc scratch [clip][tile of 64 frames][mel][64] (dct_clamp_kernel)
+  int out_tiled;             // MODE_MEL: out_r is the mfcc scratch [clip][tile of 64 frames][mel][64] (dct_clamp4_kernel)
   float amin, db_sub;
   unsigned int* clip_max;    // order-preserving uint keys of the per-clip max (log_mode)
   int* status;               // bit 0 is set when a non-finite sample reached a frame (util.valid_audio)

@@ -1,6 +1,5 @@
 // fwd_inst.cu — instantiates fwd_kernel for one transform size (compile with -DB2L_LOG2M=k).
 #include "fwd_kernel.cuh"
-#include "mel2_kernel.cuh"
 #include "internal.h"
 
 #ifndef B2L_LOG2M
@@ -41,9 +40,6 @@ cudaError_t fwd_dispatch(int op, int nw, int mode, const FwdArgs* a, int grid, s
                          int* result) {
   constexpr int M = 1 << L;
   constexpr int TPF = M >= 32 ? M / 32 : 1;
-  if constexpr (L == 10) {
-    if (nw == 3016) return run_op(mel2_kernel<L>, op, 512, a, grid, smem, st, result);   // autonomous frame groups
-  }
   if constexpr (L >= 10) {
     if (nw == 16) return by_mode<L, TPF, 16, 1>(op, mode, a, grid, smem, st, result);
     if (nw == 8) return by_mode<L, TPF, 8, 1>(op, mode, a, grid, smem, st, result);

@@ -16,19 +16,6 @@
 #include "fft_engine.cuh"
 #include "stats.cuh"
 
-#ifndef B2L_UNMIX_SHFL
-#define B2L_UNMIX_SHFL 0   // 1: real-FFT un-mix partners travel by warp shuffle where a warp owns a whole frame
-#endif
-#ifndef B2L_MEL_PVEC
-#define B2L_MEL_PVEC 4     // power values fetched per shared-memory load in the mel loop: 4 (16 bytes), 2 or 1
-#endif
-#ifndef B2L_PIPELINE
-#define B2L_PIPELINE 0     // 1: row modes fetch the next tile's operands in front of the mel phase (one rendezvous less)
-#endif
-#ifndef B2L_DEFER_BARRIER
-#define B2L_DEFER_BARRIER 2   // barrier placement of the row modes, see the comment at `release` in fwd_kernel
-#endif
-
 namespace b2l {
 
 // ------------------------------------------------------------------ mbarrier / TMA (PTX)
@@ -57,9 +44,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t phase) {
       "DONE_%=:\n\t"
       "}" ::"r"(smem_u32(bar)), "r"(phase)
       : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 // 1-D bulk copy global -> shared, completion signalled on an mbarrier (SASS: UBLKCP).
 __device__ __forceinline__ void tma_load_1d(void* dst_smem, const void* src_gmem, uint32_t bytes, uint64_t* bar) {
@@ -203,7 +187,7 @@ __global__ void __launch_bounds__(NW * 32, 1) fwd_kernel(const FwdArgs a) {
   float* s_p = reinterpret_cast<float*>(s_xall);               // P rows alias the exchange regions (MelLayout)
   const unsigned short* s_order = reinterpret_cast<const unsigned short*>(smem + a.off_melorder);
   uint64_t* s_bar = reinterpret_cast<uint64_t*>(smem + a.off_bar) + half;
-  uint64_t* s_empty = reinterpret_cast<uint64_t*>(smem + a.off_bar + 32) + half;   // "staging consumed" (B2L_DEFER_BARRIER == 3)
+  uint64_t* s_empty = reinterpret_cast<uint64_t*>(smem + a.off_bar + 32) + half;   // initialised, never waited on
 
   const int grp = htid / TPF;                  // frame group == local frame index
   const int t = htid % TPF;
@@ -269,7 +253,7 @@ __global__ void __launch_bounds__(NW * 32, 1) fwd_kernel(const FwdArgs a) {
   }
   if (htid == 0) {
     mbar_init(s_bar, 1);
-    mbar_init(s_empty, HW);
+    mbar_init(s_empty, HW);   // unused, but dropping it reschedules every instantiation: a change to measure on its own
     fence_mbar_init();
   }
   __syncthreads();
@@ -330,14 +314,10 @@ __global__ void __launch_bounds__(NW * 32, 1) fwd_kernel(const FwdArgs a) {
     const int first = (int)blockIdx.x * NH + half;
     cur = describe(first / a.tiles_per_clip, first % a.tiles_per_clip);
   }
-  uint32_t phase = 0, ephase = 0;
+  uint32_t phase = 0;
   prefetch(cur);
 
-  // B2L_PIPELINE (row modes): the operand fetch of tile i+1 is hoisted in front of the mel phase of tile i, so
-  // that the "staging consumed" barrier that follows the fetch also says "the power rows of tile i are complete"
-  // (every warp stores its row before it fetches): one rendezvous per tile less.
   constexpr bool ROWS = (MODE == MODE_MEL || MODE == MODE_STATS);
-  constexpr bool PIPE = B2L_PIPELINE && ROWS && B2L_DEFER_BARRIER == 2;
   float2 v[PPT];
   TileInfo nxt;
   // ---------------- stage a tile's sample span and turn it into windowed pass-0 operands (first stage fused in)
@@ -370,109 +350,54 @@ __global__ void __launch_bounds__(NW * 32, 1) fwd_kernel(const FwdArgs a) {
     half_sync();
     prefetch(nxt);
   };
-  if constexpr (PIPE) {
-    if (cur.clip < a.n_clips) {
-      stage_and_fetch(cur);
-      nxt = advance(cur);
-      release_staging();
-    }
-  }
 
   for (; cur.clip < a.n_clips;) {
     const int clip = cur.clip, t0 = cur.tix * FT;
-    if constexpr (!PIPE) {
-      stage_and_fetch(cur);
-      nxt = advance(cur);
-    }
-    // B0: staging buffer consumed -> prefetch the next tile behind the math.  In the modes whose power rows
-    // share the exchange regions (MEL / STATS) the same barrier also says "every warp is done with the rows
-    // of the previous tile", so it sits right before the first exchange write: the operand fetch and the
-    // register-only butterflies of pass 0 of the fast warps overlap the tail of the slow warps' mel items.
-    // B2L_DEFER_BARRIER: 0 = three barriers per tile (staging released early, "rows consumed" at the end of the
-    // tile); 1 = the two merged into one barrier before the first exchange write (late prefetch: measured 2 %
-    // slower); 2 = staging released early AND "rows consumed" deferred to just before the first exchange write.
-    // 3 = as 2, and "staging consumed" is an mbarrier on which every warp ARRIVES but only the thread that issues
-    // the bulk copy WAITS: seven of the eight warps of a half never stop there (the zero padding of edge tiles,
-    // written by all threads, moves behind the "rows consumed" barrier, which every warp passes after its fetch).
-    constexpr bool MERGED = B2L_DEFER_BARRIER == 1 && ROWS;
-    constexpr bool LATE_ROWS = B2L_DEFER_BARRIER >= 2 && ROWS;
-    constexpr bool ARRIVE_ONLY = B2L_DEFER_BARRIER == 3 && ROWS;
-    auto release = [&]() {
-      if constexpr (PIPE) {
-        // (done right after the fetch, in front of the previous tile's mel phase)
-      } else if constexpr (ARRIVE_ONLY) {
-        __syncwarp();
-        if ((htid & 31) == 0) mbar_arrive(s_empty);
-        if (htid == 0) mbar_wait(s_empty, ephase);
-        ephase ^= 1;
-        prefetch_copy(nxt);
-      } else {
-        release_staging();
-      }
-    };
-    auto rows_consumed = [&]() {
-      half_sync();
-      if constexpr (ARRIVE_ONLY) prefetch_zeros(nxt);
-    };
-    if constexpr (!MERGED) release();
+    stage_and_fetch(cur);
+    nxt = advance(cur);
+    release_staging();
 
     // ---------------- M-point complex FFT
+    // Row modes: the power rows share the exchange regions, so "every warp is done with the previous tile's rows"
+    // waits until the first exchange write — the fetch and pass 0 of fast warps overlap slow warps' mel items.
     fft_forward_tab<Cfg, true>(v, t, gbar, xbuf, tab, [&]() {
-      if constexpr (MERGED) release();
-      if constexpr (LATE_ROWS) rows_consumed();
+      if constexpr (ROWS) half_sync();
     });
-    if constexpr (MERGED && Cfg::NPASS == 1) release();
-    if constexpr (LATE_ROWS && Cfg::NPASS == 1) rows_consumed();
+    if constexpr (ROWS && Cfg::NPASS == 1) half_sync();
     // Bin pair (k, M-k), k = t + TPF*c < M/2: Z[k] is already in one of this thread's registers; only the
-    // upper half of the spectrum (indices >= M/2) has to reach its partner thread — through shared memory,
-    // or (one warp per frame, M = 1024: v[q] = Z[t + 32 q], so Z[M-k] is register 31-c of lane 32-t) with
-    // warp shuffles, which keeps 64 wavefronts per frame off the shared-memory pipe.
-    constexpr bool SHFL_UNMIX = B2L_UNMIX_SHFL && TPF == 32 && PPT == 32 && M == 1024;
+    // upper half of the spectrum (indices >= M/2) has to reach its partner thread, through shared memory.
     // un-mix addresses as one pointer per thread plus constants: measured -1.4 % (mel), -1.9 % (statistics) for
     // one-warp groups in the row modes and -0.5 % for the two-warp groups of n_fft 4096, but +6 % for the plain
     // STFT of n_fft 2048 (register allocation), which therefore keeps the index form
     constexpr bool AFFINE_UNMIX = (TPF % 32 == 0) && (TPF > 32 || MODE == MODE_MEL || MODE == MODE_STATS);
-    if constexpr (!SHFL_UNMIX) {
-      if constexpr (Cfg::NPASS > 1) group_sync<TPF>(gbar);
-      static_for<0, PPT>([&](auto S) {
-        constexpr int slot = decltype(S)::value;
-        constexpr int D = spectrum_offset<Cfg>(slot);
-        if constexpr (D >= M / 2) {
-          if constexpr (AFFINE_UNMIX && D % 32 == 0) sts_c64(smem_u32(xb_t) + 8u * (D + D / 32), v[slot]);   // xphys(t + D), D a multiple of 32
-          else sts_c64(smem_u32(xbuf) + 8u * xphys(t + D), v[slot]);
-        }
-      });
-    }
+    if constexpr (Cfg::NPASS > 1) group_sync<TPF>(gbar);
+    static_for<0, PPT>([&](auto S) {
+      constexpr int slot = decltype(S)::value;
+      constexpr int D = spectrum_offset<Cfg>(slot);
+      if constexpr (D >= M / 2) {
+        if constexpr (AFFINE_UNMIX && D % 32 == 0) sts_c64(smem_u32(xb_t) + 8u * (D + D / 32), v[slot]);   // xphys(t + D), D a multiple of 32
+        else sts_c64(smem_u32(xbuf) + 8u * xphys(t + D), v[slot]);
+      }
+    });
     tab.begin_unmix();
-    if constexpr (!SHFL_UNMIX) group_sync<TPF>(gbar);
+    group_sync<TPF>(gbar);
     auto pair_operands = [&](auto C, float2& A, float2& B) {
       constexpr int c = decltype(C)::value;
       constexpr int sa = slot_of_pair<Cfg>(c);
       static_assert(sa >= 0, "pair operand must be register resident");
       A = v[sa];
-      if constexpr (SHFL_UNMIX) {
-        const int src = (32 - t) & 31;
-        B.x = __shfl_sync(0xffffffffu, v[31 - c].x, src);
-        B.y = __shfl_sync(0xffffffffu, v[31 - c].y, src);
-        if (t == 0) B = v[c == 0 ? 0 : 32 - c];   // lane 0 pairs with itself: Z[M - 32c] = its register 32-c (Z[M] == Z[0])
+      if constexpr (AFFINE_UNMIX) {
+        // padded slot of Z[M - k], k = t + TPF*c:  K_c - xphys(t) (+ 1 in lane 0 of a warp), K_c a constant —
+        // see partner_slot; folded into one pointer per thread
+        constexpr int K = 33 * (M / 32 - 1 - (TPF / 32) * c) + 32;
+        if constexpr (c == 0) B = t == 0 ? A : xb_neg[K];   // k = 0 pairs with itself (Z[M] == Z[0])
+        else B = xb_neg[K];
       } else {
-        if constexpr (AFFINE_UNMIX) {
-          // padded slot of Z[M - k], k = t + TPF*c:  K_c - xphys(t) (+ 1 in lane 0 of a warp), K_c a constant —
-          // see partner_slot; folded into one pointer per thread
-          constexpr int K = 33 * (M / 32 - 1 - (TPF / 32) * c) + 32;
-          if constexpr (c == 0) B = t == 0 ? A : xb_neg[K];   // k = 0 pairs with itself (Z[M] == Z[0])
-          else B = xb_neg[K];
-        } else {
-          B = xbuf[partner_slot<M, TPF, c>(t)];
-          if constexpr (c == 0) {
-            if (t == 0) B = A;   // k = 0 pairs with itself (Z[M] == Z[0])
-          }
+        B = xbuf[partner_slot<M, TPF, c>(t)];
+        if constexpr (c == 0) {
+          if (t == 0) B = A;   // k = 0 pairs with itself (Z[M] == Z[0])
         }
       }
-    };
-    auto middle_bin = [&]() -> float2 {   // Z[M/2], needed by t == 0 only
-      if constexpr (SHFL_UNMIX) return v[16];
-      else return xbuf[xphys(M / 2)];
     };
 
     const int frame = t0 + grp;
@@ -494,7 +419,7 @@ __global__ void __launch_bounds__(NW * 32, 1) fwd_kernel(const FwdArgs a) {
       });
       if (t == 0) {
         float2 xa, xb;
-        float2 zc = middle_bin();
+        float2 zc = xbuf[xphys(M / 2)];   // Z[M/2]
         r2c_pair(zc, zc, make_float2(0.0f, -1.0f), xa, xb);   // W_N^(M/2) = -i
         stg_c64_if(orow + M / 2, xa, frame_ok);
       }
@@ -512,7 +437,7 @@ __global__ void __launch_bounds__(NW * 32, 1) fwd_kernel(const FwdArgs a) {
       pw[PPT] = 0.0f;
       if (t == 0) {
         float2 xa, xb;
-        float2 zc = middle_bin();
+        float2 zc = xbuf[xphys(M / 2)];   // Z[M/2]
         r2c_pair(zc, zc, make_float2(0.0f, -1.0f), xa, xb);
         pw[PPT] = sqmag(xa);
       }
@@ -558,20 +483,7 @@ __global__ void __launch_bounds__(NW * 32, 1) fwd_kernel(const FwdArgs a) {
           prow[M + 2] = 0.0f;
           prow[M + 3] = 0.0f;
         }
-        // B2: the tile's rows are complete.  Pipelined form: fetch the next tile's operands first — the barrier
-        // after that fetch is the same rendezvous.
-        if constexpr (PIPE) {
-          cur = nxt;
-          if (cur.clip < a.n_clips) {
-            stage_and_fetch(cur);
-            nxt = advance(cur);
-            release_staging();
-          } else {
-            half_sync();
-          }
-        } else {
-          half_sync();
-        }
+        half_sync();   // B2: the tile's rows are complete
         if constexpr (MODE == MODE_STATS) {
           // one warp per frame of the tile: statistics of the magnitude row (stats.cuh)
           const int hwarp = htid >> 5, lane = htid & 31;
@@ -586,8 +498,8 @@ __global__ void __launch_bounds__(NW * 32, 1) fwd_kernel(const FwdArgs a) {
           // (fp, fp + FP) over that row's padded band (host-built MelRow table: the rows of an item share
           // one trip count, start bins follow the bank rule of MelLayout, weights are zero padded and 16-byte
           // aligned).  One 16-byte weight fetch and one 16-byte power fetch per frame feed eight FMAs; no
-          // cross-lane reduction.  The items of a tile are dealt to the warps by the host (longest first,
-          // a.mel_order) because their lengths differ by an order of magnitude from the lowest to the highest rows.
+          // cross-lane reduction.  The items of a tile are dealt to the warps round-robin in row order by the host
+          // (a.mel_order): neighbouring rows, whose bands overlap in shared memory, run on warps at the same time.
           constexpr int FP = ML::FP;
           constexpr bool PAIR = ML::PAIR;
           const int hwarp = htid >> 5, lane = htid & 31;
@@ -597,7 +509,7 @@ __global__ void __launch_bounds__(NW * 32, 1) fwd_kernel(const FwdArgs a) {
           float wmax = -INFINITY;
           const float* pbase = s_p + fp * RS;
           // output row stride / base: the public [clip][mel][frame] layout, or the tiled mfcc scratch whose
-          // 64-frame tiles are contiguous 32 KB blocks for dct_clamp_kernel (t0 + fp and t0 + fp + FP share a tile)
+          // 64-frame tiles are contiguous 32 KB blocks for dct_clamp4_kernel (t0 + fp and t0 + fp + FP share a tile)
           const long long orow = a.out_tiled ? 64 : a.n_frames;
           float* obase = a.out_tiled
                              ? a.out_r + ((long long)clip * ((a.n_frames + 63) >> 6) + (t0 >> 6)) * a.n_mels * 64 + (t0 & 63) + fp
@@ -621,22 +533,7 @@ __global__ void __launch_bounds__(NW * 32, 1) fwd_kernel(const FwdArgs a) {
               const float4* pb = pa + (FP * RS) / 4;
 #pragma unroll 2
               for (; wp != wend; ++wp, ++pa, ++pb) {
-                const float4 w = *wp;
-                float4 x, y;
-                if constexpr (B2L_MEL_PVEC == 4) {
-                  x = *pa;
-                  y = *pb;
-                } else if constexpr (B2L_MEL_PVEC == 2) {
-                  const float2 x0 = reinterpret_cast<const float2*>(pa)[0], x1 = reinterpret_cast<const float2*>(pa)[1];
-                  const float2 y0 = reinterpret_cast<const float2*>(pb)[0], y1 = reinterpret_cast<const float2*>(pb)[1];
-                  x = make_float4(x0.x, x0.y, x1.x, x1.y);
-                  y = make_float4(y0.x, y0.y, y1.x, y1.y);
-                } else {
-                  const float* xa = reinterpret_cast<const float*>(pa);
-                  const float* ya = reinterpret_cast<const float*>(pb);
-                  x = make_float4(xa[0], xa[1], xa[2], xa[3]);
-                  y = make_float4(ya[0], ya[1], ya[2], ya[3]);
-                }
+                const float4 w = *wp, x = *pa, y = *pb;
                 a0 = fmaf(w.x, x.x, a0);
                 b0 = fmaf(w.x, y.x, b0);
                 a1 = fmaf(w.y, x.y, a1);
@@ -677,11 +574,10 @@ __global__ void __launch_bounds__(NW * 32, 1) fwd_kernel(const FwdArgs a) {
             if (lane == 0 && wmax > -INFINITY) atomicMax(a.clip_max + clip, float_to_key(wmax));
           }
         }
-        // deferred form: the next tile's `release` (before its first exchange write) orders the P reads
-        if constexpr (B2L_DEFER_BARRIER == 0) half_sync();
+        // (the next tile's barrier before its first exchange write orders these P reads)
       }
     }
-    if constexpr (!PIPE) cur = nxt;   // (pipelined form: already advanced in front of the mel phase)
+    cur = nxt;
   }
   if constexpr (TM) {
     tmem_fence_before_sync();
